@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W            # this repo's CUDA prover
   python bench.py --impl reference --gpus N --steps K ...  # CPU restatement of the reference
+  python bench.py ... --dump-outputs DIR                   # also write the last timed step's proofs as DIR/*.npy
 
 A "step" is one pass of the hot path over one batch of synthetic input: `--inflight` independent
 2^16-gate proofs issued concurrently (one host thread + CUDA stream each) on every rank.  Ranks
@@ -54,6 +55,22 @@ def blinders_for(i: int) -> bytes:
 
     rng = random.Random(0xB200_0000 + i)
     return b"".join(mont(rng.randrange(R_MOD)) for _ in range(14))
+
+
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(directory: str, outputs: dict):
+    """Writes every list of proofs in `outputs` as directory/<name>.npy: float32 [proofs, 1008], one byte of
+    Proof::to_bytes per element (exact in float32).  The inputs are seeded, so two builds run with the same
+    arguments can be compared output for output.  Past 64 MiB in all, each array keeps its first rows."""
+    import numpy as np
+
+    os.makedirs(directory, exist_ok=True)
+    rows = DUMP_LIMIT_BYTES // (4 * sum(len(proofs[0]) for proofs in outputs.values()))
+    for name, proofs in outputs.items():
+        a = np.frombuffer(b"".join(proofs[:rows]), dtype=np.uint8).reshape(-1, len(proofs[0]))
+        np.save(os.path.join(directory, name + ".npy"), a.astype(np.float32))
 
 
 def measured_peaks():
@@ -240,16 +257,20 @@ def run_ours(args):
     host["cpu_s_value"] = time.process_time() - cpu0
     host["after_value"] = host_cpu_state()
     launches = L.pb200_launch_count() - launches0
+    # the proofs of each timed region's last step, one per slot (later regions overwrite the buffers)
+    outputs = {"proofs": [p.raw for p in proofs]}
     cpu0 = time.process_time()
     ms_e2e = timed(args.steps, False)
     host["cpu_s_e2e"] = time.process_time() - cpu0
     host["after_e2e"] = host_cpu_state()
+    outputs["proofs_e2e"] = [p.raw for p in proofs]
     ms_synth = None
     if args.circuit == "bench":
         run_steps(1, "synth")
         t_cpu0 = time.process_time()
         ms_synth = timed(args.steps, "synth")
         cpu_s_synth = time.process_time() - t_cpu0
+        outputs["proofs_e2e_with_synthesis"] = [p.raw for p in proofs]
     # Dominant kernel (MSM bucket accumulation), timed with CUDA events on its launching stream while
     # proofs run one at a time, so the event pairs bracket the kernel alone (with several proofs in
     # flight the kernels of different streams overlap and a per-kernel duration is not meaningful).
@@ -288,6 +309,8 @@ def run_ours(args):
     if rank != 0:
         finish_dist(world)
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, outputs)
     # dominant kernel: MSM bucket accumulation.  Both hot kernels are integer-multiply bound at 256/381-bit
     # precision (SURVEY.md section 8d: ~20 MAC per algorithmic byte against a machine balance of ~2.8), so the
     # binding roofline is the ALU one; the HBM fraction is reported beside it.
@@ -604,8 +627,10 @@ def run_reference(args):
         prover.prove(blinders_for(i), arrays)
     t0 = time.time()
     for i in range(args.steps):
-        prover.prove(blinders_for(1000 + i), arrays)
+        proof = prover.prove(blinders_for(1000 + i), arrays)
     dt = time.time() - t0
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, {"proofs": [proof]})
     value = args.steps / dt
     sample = (f"each step = 1 proof of the 2^16-gate workload ({args.steps} timed after {args.warmup} warm-up); {cref.thread_policy()}; "
               "C++/OpenMP restatement (the Rust reference cannot be built here)")
@@ -637,7 +662,11 @@ def main():
     ap.add_argument("--no-proof20", action="store_true", help="skip extra.proof_2^20_ms (BASELINE.json configs[2], N = 1 only)")
     ap.add_argument("--circuit", default="bench", choices=["bench", "synthetic"],
                     help="bench = the reference's BenchCircuit<2^16> (default); synthetic = random arithmetic gates")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the proofs of each timed region's last step as DIR/<name>.npy (float32 bytes)")
     args = ap.parse_args()
+    if args.steps is not None and args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.impl == "reference":
         args.steps = args.steps if args.steps is not None else 3
         args.warmup = args.warmup if args.warmup is not None else 1
